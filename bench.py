@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — pairs/s of RoMa dense match() (+ sample()) at 560 -> 864 on B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|fp32_simt|fp16|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp32|fp32_simt|fp16|bf16] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic input: `roma_outdoor(...).match()` on
@@ -19,6 +19,13 @@ no data-path collective — pairs are independent, SURVEY §8e).  Prints ONE JSO
              the 1e-4 bar: "fp32" = fp32-class GEMMs on tcgen05 from split-fp16 operand pairs (DESIGN.md §2)
   fast_mode  the same workload in the reference's CUDA autocast regime (fp16 operands), reported beside it with its error
   cpu_baseline  the CPU oracle (a port of the reference's fp32 CPU path) on this box's host cores, one pair
+--dump-outputs DIR writes what the last timed step returned to its caller on rank 0 as float32 .npy files: warp and certainty
+(rank 0's match() results; the whole gathered batch when N > 1 scatters it) and sample_matches, sample_certainty (only the pairs
+rank 0 sampled itself, so fewer pairs than warp when the batch is sharded).  Inputs are seeded and torch's generator is seeded
+before the timed steps, so two builds run with the same arguments can be compared file by file.  The samples are reproducible
+with one pair per step (the default): sample() calls share one pinned seed buffer, so with several pairs per step an earlier
+call can read a later call's seeds.  Above DUMP_LIMIT bytes in all, every file keeps the same seeded subset of its rows (pixels
+of warp / certainty, samples), flattened to [rows] or [rows, 4].
 --impl reference times that CPU path alone (the reference itself is pure Python/PyTorch and does not travel
 to the GPU box; `oracle/` is its validated restatement, bit-exact against it in the build container).
 """
@@ -35,6 +42,25 @@ sys.path.insert(0, ROOT)
 
 COARSE, UPSAMPLE = 560, 864
 FLOP_PER_PAIR = 6.58e12          # SURVEY §6 (FlopCounterMode + analytic attention/solves)
+DUMP_LIMIT = 64 * 10 ** 6       # bytes of --dump-outputs in all
+
+
+def dump_outputs(path, outputs):
+    """Writes {name: tensor} as path/<name>.npy in float32.  When the total exceeds DUMP_LIMIT, each array is cut to the same
+    fraction of its rows (a 4-vector of warp / sample_matches, one value of the certainties), drawn with a fixed seed: arrays
+    with the same row count (warp and certainty; the two sample outputs) keep the same rows."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        frac = (DUMP_LIMIT - 4096 * len(arrays)) / total                 # room for the .npy headers
+        for k, a in arrays.items():
+            rows = a.reshape(-1, 4) if k in ("warp", "sample_matches") else a.reshape(-1)
+            keep = np.sort(np.random.default_rng(0).choice(len(rows), int(len(rows) * frac), replace=False))
+            arrays[k] = rows[keep]
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 def load_peaks():
@@ -421,12 +447,15 @@ def run_ours(args):
     sample_calls = [0]
 
     sample_host = {}                                  # pinned read-back buffers of the samples, per pair slot of a step
+    dump_step = {}                                    # --dump-outputs: this rank's results of the current headline step
 
     def sample_batch(warp, cert, to_host=False):
         if args.no_sample:
             return
         for i in range(warp.shape[0]):
             m, c = model.sample(warp[i], cert[i], num=10000)
+            if "samples" in dump_step:
+                dump_step["samples"].append((m, c))
             if to_host:
                 # asynchronous read-back into pinned memory on the step's stream: no host synchronisation inside a step, so the host
                 # queues the next step while this one runs (a blocking .cpu() here exposed ~0.2 ms of launch latency per step)
@@ -555,9 +584,23 @@ def run_ours(args):
     sampler = ClockSampler(local)
     sampler.start()
     time.sleep(0.3)
+
+    def dump_step_device():
+        dump_step["samples"] = []
+        dump_step["out"] = step_device()
+    if args.dump_outputs:
+        torch.manual_seed(0)                                  # sample() draws its seeds from torch's CPU generator
     launches0 = cabi.kernel_launches() + model.graph_launches
-    ms = timed(step_device, args.steps)                       # headline: device side replayed as a CUDA graph
+    ms = timed(dump_step_device if args.dump_outputs else step_device, args.steps)      # headline: device side replayed as a CUDA graph
     launches = cabi.kernel_launches() + model.graph_launches - launches0
+    if args.dump_outputs:
+        if rank == 0:
+            outputs = dict(zip(("warp", "certainty"), dump_step["out"]))
+            if dump_step["samples"]:
+                outputs["sample_matches"] = torch.cat([m for m, _ in dump_step["samples"]])
+                outputs["sample_certainty"] = torch.cat([c for _, c in dump_step["samples"]])
+            dump_outputs(args.dump_outputs, outputs)
+        dump_step.clear()
     # second timed region, same workload, eager launches with a CUDA-event pair around every GEMM launch and every
     # pipeline stage (events cannot be read back from inside a replayed graph): feeds `roofline` and the stage table
     eng.gemm_profile, eng.profile = [], {}
@@ -820,7 +863,10 @@ def main():
     ap.add_argument("--no-scatter", action="store_true", help="N > 1: every rank on its own resident pairs (no NCCL scatter / gather in the timed region)")
     ap.add_argument("--no-sample", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's warp, certainty and samples to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "torch_cuda":
         import torch
         if int(os.environ.get("RANK", "0")) == 0:

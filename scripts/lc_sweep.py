@@ -8,7 +8,6 @@ dev = torch.device("cuda:0")
 out = {}
 for mode in ("engine", "per_pixel", "tile_all"):
     out[mode] = bench.local_corr_flow_sweep(dev, "fp32", mode)
-peak = json.load(open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "MEASURED_PEAKS.json")))
 print(json.dumps(out))
 for k, v in out.items():
     for kind, r in v.items():

@@ -185,12 +185,15 @@ def test_cabi_call_validates_tensors():
     with pytest.raises(TypeError):
         cabi.call("romab200_gemm", "rb_gemm_args", not_a_field=1)
     # dtype / contiguity / size rules, exercised on the validator itself with the device check satisfied by a stand-in
+    # (on the current CUDA device when there is one)
+    index = torch.cuda.current_device() if torch.cuda.is_available() else None
+
     class FakeCuda(torch.Tensor):
         is_cuda = True
 
         @property
         def device(self):
-            return type("D", (), {"index": None})()
+            return type("D", (), {"index": index})()
     def fake(t):
         return t.as_subclass(FakeCuda)
     half, f32 = fake(torch.zeros(8, 8, dtype=torch.float16)), fake(torch.zeros(8, 8))

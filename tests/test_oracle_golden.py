@@ -21,12 +21,24 @@ def _oracle(weights, g):
     return RomaOracle(weights[0], weights[1], coarse, up or coarse, symmetric=bool(sym), upsample_preds=bool(upp))
 
 
-def _check(warp, cert, g, step=1):
+def _check(warp, cert, g):
+    """Max-abs error on the golden's pixels (every meta[6]-th row and column); over the whole tensors, the mean errors of the
+    sum and the absolute sum (float64 checksums in the golden), which the max-abs error over all pixels bounds."""
+    step = int(g["meta"][6])
     w = warp[:, ::step, ::step].numpy()
     c = cert[:, ::step, ::step].numpy()
     assert w.shape == g["warp"].shape and c.shape == g["certainty"].shape
     assert np.abs(w - g["warp"]).max() <= TOL
     assert np.abs(c - g["certainty"]).max() <= TOL
+    for t, key in ((warp, "warp_checksum"), (cert, "certainty_checksum")):
+        t = t.double()
+        assert abs(t.sum().item() - g[key][0]) <= TOL * t.numel() and abs(t.abs().sum().item() - g[key][1]) <= TOL * t.numel()
+
+
+def _stage(t, g, key):
+    """The golden's subset of stage tensor `key` [B, C, H, W] (channel / spatial steps in `key_step`)."""
+    c, s = (int(v) for v in g[f"{key}_step"])
+    return t[:, ::c, ::s, ::s].numpy()
 
 
 @pytest.mark.parametrize("name", ["small_sym_up", "small_nosym_up", "small_sym_noup", "small_b2_sym_up"])
@@ -36,6 +48,8 @@ def test_oracle_matches_reference_small(weights, name):
     orc = _oracle(weights, g)
     A, B, Ah, Bh = synthetic.make_pair(batch, coarse, up if upp else None, seed)
     warp, cert = orc.match(A, B, Ah, Bh)
+    h = up if upp else coarse
+    assert warp.shape == (batch, h, h * (2 if sym else 1), 4) and cert.shape == warp.shape[:3]
     _check(warp, cert, g)
     assert warp.dtype == torch.float32 and cert.dtype == torch.float32
 
@@ -57,11 +71,12 @@ def test_oracle_stage_tensors(weights):
     A, B, Ah, Bh = synthetic.make_pair(1, 112, 168, 1)
     orc.match(A, B, Ah, Bh)
     t = orc.trace
-    assert np.abs(t["gp.mu"].numpy() - g["gp_mu"]).max() <= TOL
-    assert np.abs(t["cls"].numpy() - g["cls_and_cert"][:, :-1]).max() <= 1e-3     # logits are O(40)
+    assert np.abs(_stage(t["gp.mu"], g, "gp_mu") - g["gp_mu"]).max() <= TOL
+    # the kept classes are those of cls_and_cert but its last (certainty) channel
+    assert np.abs(_stage(t["cls"], g, "cls_and_cert") - g["cls_and_cert"][:, :-1]).max() <= 1e-3     # logits are O(40)
     for s in (16, 8, 4, 2, 1):
-        assert np.abs(t[f"lo.delta{s}"].numpy() - g[f"delta{s}"]).max() <= TOL * 10
-        assert np.abs(t[f"lo.proj{s}.x"].numpy() - g[f"proj{s}"]).max() <= TOL
+        assert np.abs(_stage(t[f"lo.delta{s}"], g, f"delta{s}") - g[f"delta{s}"]).max() <= TOL * 10
+        assert np.abs(_stage(t[f"lo.proj{s}.x"], g, f"proj{s}") - g[f"proj{s}"]).max() <= TOL
 
 
 def test_oracle_pil_route(weights):
@@ -94,6 +109,6 @@ def test_oracle_matches_reference_full(weights):
     orc = _oracle(weights, g)
     A, B, Ah, Bh = synthetic.make_pair(1, 560, 864, 1)
     warp, cert = orc.match(A, B, Ah, Bh)
-    _check(warp, cert, g, step=8)
+    _check(warp, cert, g)
     assert abs(warp.double().sum().item() - g["warp_checksum"][0]) <= 1e-3 * max(1.0, abs(g["warp_checksum"][0]))
     assert abs(cert.double().abs().sum().item() - g["certainty_checksum"][1]) <= 1e-4 * g["certainty_checksum"][1]
