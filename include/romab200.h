@@ -264,10 +264,15 @@ int romab200_refiner_block_small(const rb_refiner_block_small_args* args, void* 
 
 /* Fused ConvRefiner block for the stride-2 maps (C = 144): depthwise 5x5 + BN + ReLU on the CUDA cores feeding a
  * tcgen05 pointwise GEMM whose weights stay resident in shared memory; one read + one write of the map.
- * in/out [batch, h, w, ld] 16-bit (in != out); dw_weight [25][ldw] fp32 (BN folded), pw_weight [144][ld_pw] 16-bit. */
+ * in/out [batch, h, w, ld] (in != out); dw_weight [25][ldw] fp32 (BN folded).
+ * dtype RB_F16 / RB_BF16: 16-bit maps, pw_weight [144][ld_pw] in the same type.
+ * dtype RB_F32: fp32 maps (ld % 4 == 0, ldw even), pointwise weights as an RB_F16S pair: pw_weight = hi plane,
+ * pw_weight_lo = lo plane, both [144][ld_pw] fp16.  The result is bit-identical to romab200_dwconv5x5_relu (RB_F32 in,
+ * RB_F16S out) followed by the split-fp16 romab200_gemm with the pointwise bias. */
 typedef struct {
     const void* in; void* out; int64_t ld; const float* dw_weight; int64_t ldw; const float* dw_bias;
     const void* pw_weight; int64_t ld_pw; const float* pw_bias; int32_t batch, h, w, c; int32_t dtype;
+    const void* pw_weight_lo;   /* dtype == RB_F32 only */
 } rb_refiner_block_c144_args;
 int romab200_refiner_block_c144(const rb_refiner_block_c144_args* args, void* stream);
 

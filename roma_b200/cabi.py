@@ -103,7 +103,7 @@ def _stream():
 launch_count = 0      # number of C-ABI calls made (bench.py reports kernel launches from it)
 
 # ---- argument validation: the C ABI takes raw pointers, so a tensor of the wrong dtype / device / layout would be silent garbage.
-# For every struct: tensor field -> the field that carries its dtype code (or a fixed torch dtype).
+# For every struct: tensor field -> the field that carries its dtype code (or a fixed torch dtype, or a function of the call's fields).
 _CODE_DTYPE = {RB_F32: torch.float32, RB_F16: torch.float16, RB_BF16: torch.bfloat16, RB_F16S: torch.float16}
 _F32 = torch.float32
 _FIELD_DTYPES = {
@@ -127,7 +127,9 @@ _FIELD_DTYPES = {
     "rb_local_corr_warp_args": {"f0": _F32, "f1": _F32, "warp": _F32, "out": _F32},
     "rb_dwconv_args": {"in": "dtype", "weight": _F32, "bias": _F32, "out_lo": torch.float16},
     "rb_refiner_block_small_args": {"in": "dtype", "out": "dtype", "dw_weight": _F32, "dw_bias": _F32},
-    "rb_refiner_block_c144_args": {"in": "dtype", "out": "dtype", "dw_weight": _F32, "dw_bias": _F32, "pw_weight": "dtype", "pw_bias": _F32},
+    "rb_refiner_block_c144_args": {"in": "dtype", "out": "dtype", "dw_weight": _F32, "dw_bias": _F32, "pw_bias": _F32, "pw_weight_lo": torch.float16,
+                                   # fp32 maps take the pointwise weights as an RB_F16S pair (pw_weight = hi plane)
+                                   "pw_weight": lambda kw: torch.float16 if kw.get("dtype") == RB_F32 else _CODE_DTYPE.get(kw.get("dtype"))},
     "rb_refiner_tail_args": {"d": "dtype", "weight": _F32, "bias": _F32, "state": _F32, "delta_out": _F32},
     "rb_resize_args": {"in": _F32, "out": _F32},
     "rb_match_epilogue_args": {"state": _F32, "coarse_state": _F32, "warp": _F32, "cert": _F32, "grid_x": _F32, "grid_y": _F32},
@@ -170,6 +172,8 @@ def _validate(fn_name, struct_name, kw):
         want = table.get(k)
         if isinstance(want, str):
             want = _CODE_DTYPE.get(kw.get(want))
+        elif callable(want) and not isinstance(want, torch.dtype):
+            want = want(kw)
         if want is not None and v.dtype != want:
             raise RuntimeError(f"{fn_name}: argument `{k}` has dtype {v.dtype}, the call describes it as {want}")
         if k in mins and v.numel() < mins[k]:

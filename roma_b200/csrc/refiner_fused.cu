@@ -9,6 +9,8 @@
 //   * 1 thread issues 9 tcgen05.mma (M=128, N=144, K=16) against the pointwise weights, which were TMA-loaded into
 //     shared memory once and stay resident;
 //   * 4 epilogue warps read the fp32 accumulator from TMEM (double-buffered), add the bias and store 16-bit rows.
+// refiner_block_c144_split_kernel (below) is the same block on fp32 maps with split-fp16 pointwise operands (parity mode),
+// bit-identical to the depthwise kernel + split GEMM pair it replaces.
 #include "common.cuh"
 #include <cuda.h>
 
@@ -84,15 +86,23 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
-__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
+// UMMA shared-memory descriptor; layout 2 = SWIZZLE_128B, 4 = SWIZZLE_64B
+__device__ __forceinline__ uint64_t smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout = 2) {
     uint64_t d = 0;
     d |= (uint64_t)((saddr >> 4) & 0x3FFF);
     d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
     d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
     d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
+    d |= (uint64_t)layout << 61;
     return d;
 }
+__device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, const void* smem_src, int c0, int c1, int c2, int c3) {
+    asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
+                 ::"l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 }  // namespace fz
 
 #ifdef RB_FZ_CLK
@@ -295,6 +305,256 @@ __global__ void __launch_bounds__(FZ_THREADS, 1) refiner_block_c144_kernel(const
     if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, 512); }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// The same block on fp32 maps (parity mode), with the pointwise GEMM on split-fp16 operand pairs: one kernel in place of
+// dwconv5x5_relu_tma_kernel<float> (fp32 map -> RB_F16S pair in memory) followed by gemm_tc_kernel<144, SPLIT>.  Both
+// halves do exactly the arithmetic of those two kernels, so the output is bit-identical to theirs:
+//   * depthwise: accumulator = bias, 25 packed FFMA2 per output in (ky, kx) order, ReLU, hi = fp16(x), lo = fp16((x - hi) * 2^11);
+//   * pointwise: per k-step of 16, acc0 += A_hi.B_hi, then acc1 += A_hi.B_lo and acc1 += A_lo.B_hi, k ascending (9 steps);
+//   * epilogue: acc0 + acc1 * 2^-11 (one fmaf), then + bias, stored as fp32.
+// The fp32 window of all 144 channels (138 KB) does not fit beside the resident weights, so a tile is streamed in five
+// 32-channel chunks (the last 16 wide: its upper half is the tensor map's zero fill and is never read by an MMA):
+//   * warp 5, one thread: TMA-loads the 12 x 20 pixel x 32 channel fp32 window of a chunk into a 3-stage ring;
+//   * warps 6-13 (256 threads = 16 channel pairs x 4 row pairs x 4 column quarters, 2 x 4 outputs each) run the depthwise
+//     stage of the chunk and write its hi / lo planes into a 64B-swizzled K-major A stage (two stages);
+//   * warp 0, one thread: issues the 2 (last chunk: 1) k-steps of the chunk as soon as its A stage is written;
+//   * warps 1-4: drain the two accumulators (288 of 512 TMEM columns: single-buffered), release TMEM after the last load, and
+//     store fp32 rows through TMA (16 channels x 16 pixels x 2 rows per store; image borders clipped by the tensor map).
+//     This overlaps the depthwise stage of the first chunks of the next tile.
+// Shared memory (bytes): B hi + lo, 5 chunks x 144 rows x 64 B each   92160
+//                        A hi + lo, 2 stages x 128 rows x 64 B each   32768
+//                        input windows, 3 x 12 x 20 x 32 x 4          92160
+//                        epilogue staging, 4 warps x 2 KB              8192
+//                        bias, barriers, TMEM slot, 1 KB alignment     1792   -> 227072 of 232448, one CTA per SM
+// The depthwise taps (14 KB) are read per chunk from global memory through L1; there is no room for them here.
+constexpr int FS_CH = 32, FS_NCHUNK = 5, FS_WIN_STAGES = 2 + 1;
+constexpr int FS_DW_THREADS = 256;
+constexpr int FS_THREADS = 32 + 128 + 32 + FS_DW_THREADS;   // warp 0: weights + MMA, warps 1-4: epilogue, warp 5: input TMA, warps 6-13: depthwise
+constexpr int FS_WIN_BYTES = FZ_IH * FZ_IW * FS_CH * 4;     // 30720
+constexpr int FS_B_CHUNK = FZ_C * FS_CH * 2;                // 9216: 144 rows x 64 B
+constexpr int FS_B_PLANE = FS_NCHUNK * FS_B_CHUNK;          // 46080
+constexpr int FS_A_PLANE = 128 * FS_CH * 2;                 // 8192
+constexpr int FS_A_STAGE = 2 * FS_A_PLANE;                  // hi + lo
+constexpr int FS_OUT_WARP = 32 * 16 * 4;                    // 2048: 32 pixels x 16 fp32 channels
+constexpr int FS_OFF_A = 2 * FS_B_PLANE;
+constexpr int FS_OFF_WIN = FS_OFF_A + 2 * FS_A_STAGE;
+constexpr int FS_OFF_OUT = FS_OFF_WIN + FS_WIN_STAGES * FS_WIN_BYTES;
+constexpr int FS_OFF_BIAS = FS_OFF_OUT + 4 * FS_OUT_WARP;
+constexpr int FS_OFF_BAR = FS_OFF_BIAS + FS_NCHUNK * FS_CH * 4;
+constexpr int FS_SMEM = FS_OFF_BAR + 128 + 1024;
+static_assert(FS_SMEM <= 232448, "shared memory budget");
+
+struct FusedSplitParams {
+    const float* dw_w; int64_t ldw; const float* dw_b; const float* pw_b;
+    int H, W, tiles_x, tiles_y, total_tiles;
+};
+
+__global__ void __launch_bounds__(FS_THREADS, 1)
+refiner_block_c144_split_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
+                                const __grid_constant__ CUtensorMap map_in, const __grid_constant__ CUtensorMap map_out, const FusedSplitParams p) {
+    rb::pdl_wait();
+    using namespace fz;
+    extern __shared__ uint8_t smem_raw[];
+    uint8_t* smem = smem_raw + ((1024u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 1023u)) & 1023u);
+    uint8_t* sB = smem;                                   // [hi | lo][chunk][144 rows][64 B], 64B-swizzled
+    uint8_t* sA = smem + FS_OFF_A;                        // [stage][hi | lo][128 rows][64 B], 64B-swizzled
+    uint8_t* sWin = smem + FS_OFF_WIN;                    // [stage][12 rows][20 pixels][32 channels] fp32
+    uint8_t* sOut = smem + FS_OFF_OUT;                    // [epilogue warp][32 pixels][16 channels] fp32
+    float* s_bias = reinterpret_cast<float*>(smem + FS_OFF_BIAS);   // [160], zero beyond 144
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FS_OFF_BAR);
+    uint64_t* w_full = bars;              // pointwise weights landed
+    uint64_t* win_full = bars + 1;        // [3] input window landed (TMA transaction bytes)
+    uint64_t* win_empty = bars + 4;       // [3] depthwise warps have read it (8 warp arrivals)
+    uint64_t* a_full = bars + 7;          // [2] A stage written (8 warp arrivals)
+    uint64_t* a_empty = bars + 9;         // [2] MMAs that read it retired
+    uint64_t* t_full = bars + 11;         // accumulators complete
+    uint64_t* t_empty = bars + 12;        // accumulators drained (4 warp arrivals)
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 13);
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) {
+        mbar_init(w_full, 1);
+        for (int s = 0; s < FS_WIN_STAGES; ++s) { mbar_init(&win_full[s], 1); mbar_init(&win_empty[s], FS_DW_THREADS / 32); }
+        for (int s = 0; s < 2; ++s) { mbar_init(&a_full[s], FS_DW_THREADS / 32); mbar_init(&a_empty[s], 1); }
+        mbar_init(t_full, 1); mbar_init(t_empty, 4);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 1) tmem_alloc(tmem_slot, 512);
+    for (int i = threadIdx.x; i < FS_NCHUNK * FS_CH; i += FS_THREADS) s_bias[i] = i < FZ_C ? p.pw_b[i] : 0.f;
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+    const int tiles_per_img = p.tiles_x * p.tiles_y;
+
+    if (warp == 0) {
+        if (lane == 0) {
+            // pointwise weights: both planes as five 32-wide k-chunks, loaded once for the whole persistent kernel
+            mbar_expect_tx(w_full, 2 * FS_B_PLANE);
+            for (int c = 0; c < FS_NCHUNK; ++c) {
+                tma_load_2d(sB + c * FS_B_CHUNK, &map_w_hi, w_full, c * FS_CH, 0);
+                tma_load_2d(sB + FS_B_PLANE + c * FS_B_CHUNK, &map_w_lo, w_full, c * FS_CH, 0);
+            }
+            const uint32_t idesc = (1u << 4) | ((uint32_t)(FZ_C >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);   // f32 += f16 x f16, K-major
+            mbar_wait(w_full, 0);
+            const uint32_t a_addr = smem_u32(sA), b_addr = smem_u32(sB);
+            uint32_t it = 0, j = 0;
+            for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++it) {
+                mbar_wait(t_empty, (it & 1) ^ 1);
+                tc_fence_after();
+#pragma unroll
+                for (int c = 0; c < FS_NCHUNK; ++c, ++j) {
+                    const uint32_t s = j & 1;
+                    mbar_wait(&a_full[s], (j >> 1) & 1);
+                    tc_fence_after();
+                    const uint32_t a_hi = a_addr + s * FS_A_STAGE, a_lo = a_hi + FS_A_PLANE;
+                    const uint32_t b_hi = b_addr + c * FS_B_CHUNK, b_lo = b_hi + FS_B_PLANE;
+#pragma unroll
+                    for (int ks = 0; ks < 2; ++ks) {
+                        if (2 * c + ks < FZ_C / 16) {          // k-steps beyond K = 144 are skipped, as in gemm_tc
+                            const uint32_t accum = (c | ks) != 0;
+                            const uint64_t dah = smem_desc(a_hi + 32 * ks, 16, 512, 4), dal = smem_desc(a_lo + 32 * ks, 16, 512, 4);
+                            const uint64_t dbh = smem_desc(b_hi + 32 * ks, 16, 512, 4), dbl = smem_desc(b_lo + 32 * ks, 16, 512, 4);
+                            umma_f16(tmem_base, dah, dbh, idesc, accum);
+                            umma_f16(tmem_base + FZ_C, dah, dbl, idesc, accum);
+                            umma_f16(tmem_base + FZ_C, dal, dbh, idesc, 1u);
+                        }
+                    }
+                    umma_commit(&a_empty[s]);
+                }
+                umma_commit(t_full);
+            }
+        }
+    } else if (warp <= 4) {
+        // ===== epilogue: TMEM -> acc0 + acc1 * 2^-11 + bias -> fp32 rows through TMA stores =====
+        const int q = warp & 3;                            // TMEM lane quarter = pixels 32q .. 32q + 31 = tile rows 2q, 2q + 1
+        uint8_t* stage = sOut + (warp - 1) * FS_OUT_WARP;
+        uint32_t it = 0;
+        for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++it) {
+            const int img = tile / tiles_per_img, r = tile - img * tiles_per_img;
+            const int ty = r / p.tiles_x, tx = r - ty * p.tiles_x;
+            const int y0 = ty * FZ_TH + 2 * q;
+            mbar_wait(t_full, it & 1);
+            tc_fence_after();
+#pragma unroll 1
+            for (int cb = 0; cb < FZ_C; cb += 32) {
+                float v[32], w[32];
+                tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + cb, v);
+                tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + FZ_C + cb, w);
+                if (cb + 32 >= FZ_C) {                         // last chunk read: the MMA thread may start the next tile
+                    tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(t_empty);
+                }
+#pragma unroll
+                for (int k = 0; k < 32; ++k) v[k] = fmaf(w[k], 1.0f / 2048.0f, v[k]);
+#pragma unroll
+                for (int k = 0; k < 8; ++k) {
+                    const float4 b4 = *reinterpret_cast<const float4*>(&s_bias[cb + 4 * k]);
+                    v[4 * k] += b4.x; v[4 * k + 1] += b4.y; v[4 * k + 2] += b4.z; v[4 * k + 3] += b4.w;
+                }
+                if (y0 >= p.H) continue;                       // warp-uniform: both rows below the image
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    if (cb + 16 * h >= FZ_C) break;
+                    if (lane == 0) bulk_wait_read();           // the previous store has read the staging buffer
+                    __syncwarp();
+#pragma unroll
+                    for (int k = 0; k < 4; ++k)
+                        *reinterpret_cast<float4*>(stage + lane * 64 + 16 * k) = make_float4(v[16 * h + 4 * k], v[16 * h + 4 * k + 1], v[16 * h + 4 * k + 2], v[16 * h + 4 * k + 3]);
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    __syncwarp();
+                    if (lane == 0) { tma_store_4d(&map_out, stage, cb + 16 * h, tx * FZ_TW, y0, img); bulk_commit(); }
+                }
+            }
+        }
+        if (lane == 0) bulk_wait_all();
+        __syncwarp();
+    } else if (warp == 5) {
+        // ===== input loader: one TMA box per (tile, chunk), 3 windows in flight =====
+        if (lane == 0) {
+            uint32_t j = 0;
+            for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
+                const int img = tile / tiles_per_img, r = tile - img * tiles_per_img;
+                const int ty = r / p.tiles_x, tx = r - ty * p.tiles_x;
+                for (int c = 0; c < FS_NCHUNK; ++c, ++j) {
+                    const uint32_t s = j % FS_WIN_STAGES;
+                    if (j >= FS_WIN_STAGES) mbar_wait(&win_empty[s], (j / FS_WIN_STAGES - 1) & 1);
+                    mbar_expect_tx(&win_full[s], FS_WIN_BYTES);
+                    tma_load_4d(sWin + s * FS_WIN_BYTES, &map_in, &win_full[s], c * FS_CH, tx * FZ_TW - 2, ty * FZ_TH - 2, img);
+                }
+            }
+        }
+    } else {
+        // ===== depthwise: thread = (channel pair, 2 output rows, 4 output columns) of the chunk =====
+        const int t = threadIdx.x - 192;                   // 0 .. 255
+        const int pr = t & 15, xq = (t >> 4) & 3, rg = t >> 6;
+        const int sw_chunk = pr >> 2, inb = (pr & 3) * 4;  // 16-byte chunk and byte of this pair in a 64-byte A row
+        uint32_t j = 0;
+        for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
+#pragma unroll 1
+            for (int c = 0; c < FS_NCHUNK; ++c, ++j) {
+                const int ch = c * FS_CH + 2 * pr;
+                const bool ok = ch < FZ_C;                 // the upper half of the last chunk computes zeros that no MMA reads
+                float2 wv[25];
+#pragma unroll
+                for (int k = 0; k < 25; ++k) wv[k] = ok ? __ldg(reinterpret_cast<const float2*>(p.dw_w + k * p.ldw + ch)) : make_float2(0.f, 0.f);
+                const float2 bv = ok ? __ldg(reinterpret_cast<const float2*>(p.dw_b + ch)) : make_float2(0.f, 0.f);
+                const uint32_t s = j % FS_WIN_STAGES;
+                mbar_wait(&win_full[s], (j / FS_WIN_STAGES) & 1);
+                const float* win = reinterpret_cast<const float*>(sWin + s * FS_WIN_BYTES);
+                float2 acc[2][4];
+#pragma unroll
+                for (int rr = 0; rr < 2; ++rr)
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) acc[rr][i] = bv;
+#pragma unroll
+                for (int iy = 0; iy < 6; ++iy) {
+#pragma unroll
+                    for (int ix = 0; ix < 8; ++ix) {
+                        const float2 v = *reinterpret_cast<const float2*>(&win[((2 * rg + iy) * FZ_IW + 4 * xq + ix) * FS_CH + 2 * pr]);
+#pragma unroll
+                        for (int rr = 0; rr < 2; ++rr) {
+                            const int ky = iy - rr;
+                            if (ky >= 0 && ky < 5) {
+#pragma unroll
+                                for (int kx = 0; kx < 5; ++kx) {
+                                    const int ox = ix - kx;
+                                    if (ox >= 0 && ox < 4) acc[rr][ox] = __ffma2_rn(wv[ky * 5 + kx], v, acc[rr][ox]);
+                                }
+                            }
+                        }
+                    }
+                }
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&win_empty[s]);
+                const uint32_t as = j & 1;
+                mbar_wait(&a_empty[as], ((j >> 1) & 1) ^ 1);   // the MMAs of chunk j - 2 no longer read this A stage
+                uint8_t* a_hi = sA + as * FS_A_STAGE;
+#pragma unroll
+                for (int rr = 0; rr < 2; ++rr) {
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) {
+                        const int m = (2 * rg + rr) * FZ_TW + 4 * xq + i;
+                        __half hi[2], lo[2];
+                        split_f16s(fmaxf(acc[rr][i].x, 0.f), hi[0], lo[0]);
+                        split_f16s(fmaxf(acc[rr][i].y, 0.f), hi[1], lo[1]);
+                        const int off = m * 64 + ((sw_chunk ^ ((m >> 1) & 3)) << 4) + inb;
+                        *reinterpret_cast<uint32_t*>(a_hi + off) = *reinterpret_cast<uint32_t*>(hi);
+                        *reinterpret_cast<uint32_t*>(a_hi + FS_A_PLANE + off) = *reinterpret_cast<uint32_t*>(lo);
+                    }
+                }
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                __syncwarp();
+                if (lane == 0) mbar_arrive(&a_full[as]);
+            }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, 512); }
+}
+
 typedef CUresult (*EncodeTiledFnFz)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                     const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -309,12 +569,58 @@ extern "C" int romab200_debug_fzclk(long long* out, int reset) {
 }
 #endif
 
+// fp32 maps, split-fp16 pointwise weights (pw_weight = hi plane, pw_weight_lo = lo plane)
+static int refiner_block_c144_split(const rb_refiner_block_c144_args* a, cudaStream_t st, EncodeTiledFnFz enc) {
+    RB_REQUIRE(a->ld % 4 == 0 && a->ld >= FZ_C && ((uintptr_t)a->in) % 16 == 0 && ((uintptr_t)a->out) % 16 == 0 && a->in != a->out,
+               "refiner_block_c144: bad fp32 activation layout");
+    RB_REQUIRE(a->pw_weight_lo && ((uintptr_t)a->pw_weight_lo) % 16 == 0, "refiner_block_c144: fp32 maps need the lo plane of the split weights (pw_weight_lo)");
+    RB_REQUIRE(a->ldw % 2 == 0 && ((uintptr_t)a->dw_weight) % 8 == 0 && ((uintptr_t)a->dw_bias) % 8 == 0, "refiner_block_c144: bad depthwise weight layout");
+    CUtensorMap map_w[2];        // weight planes [144 x ld_pw] fp16: boxes of 32 (k) x 144 (n), 64B-swizzled K-major
+    for (int i = 0; i < 2; ++i) {
+        cuuint64_t dims[2] = {(cuuint64_t)FZ_C, (cuuint64_t)FZ_C};
+        cuuint64_t strides[1] = {(cuuint64_t)a->ld_pw * 2};
+        cuuint32_t box[2] = {(cuuint32_t)FS_CH, (cuuint32_t)FZ_C};
+        cuuint32_t estr[2] = {1, 1};
+        CUresult r = enc(&map_w[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(i ? a->pw_weight_lo : a->pw_weight), dims, strides, box, estr,
+                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        RB_REQUIRE(r == CUDA_SUCCESS, "refiner_block_c144: cuTensorMapEncodeTiled (weights) failed with %d", (int)r);
+    }
+    // activations [B, H, W, 144] fp32 with pitch ld: input boxes 12 x 20 pixels x 32 channels (borders and the channel tail zero-filled),
+    // output boxes 2 x 16 pixels x 16 channels (clipped at the borders)
+    CUtensorMap map_in, map_out;
+    cuuint64_t d4[4] = {(cuuint64_t)FZ_C, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->batch};
+    cuuint64_t s4[3] = {(cuuint64_t)a->ld * 4, (cuuint64_t)a->w * a->ld * 4, (cuuint64_t)a->h * a->w * a->ld * 4};
+    cuuint32_t e4[4] = {1, 1, 1, 1};
+    cuuint32_t bin[4] = {(cuuint32_t)FS_CH, (cuuint32_t)FZ_IW, (cuuint32_t)FZ_IH, 1};
+    CUresult r = enc(&map_in, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<void*>(a->in), d4, s4, bin, e4, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    RB_REQUIRE(r == CUDA_SUCCESS, "refiner_block_c144: cuTensorMapEncodeTiled (input) failed with %d", (int)r);
+    cuuint32_t bout[4] = {16, (cuuint32_t)FZ_TW, 2, 1};
+    r = enc(&map_out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, a->out, d4, s4, bout, e4, CU_TENSOR_MAP_INTERLEAVE_NONE,
+            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    RB_REQUIRE(r == CUDA_SUCCESS, "refiner_block_c144: cuTensorMapEncodeTiled (output) failed with %d", (int)r);
+    FusedSplitParams p;
+    p.dw_w = a->dw_weight; p.ldw = a->ldw; p.dw_b = a->dw_bias; p.pw_b = a->pw_bias;
+    p.H = a->h; p.W = a->w; p.tiles_x = (a->w + FZ_TW - 1) / FZ_TW; p.tiles_y = (a->h + FZ_TH - 1) / FZ_TH;
+    const long long total = (long long)p.tiles_x * p.tiles_y * a->batch;
+    RB_REQUIRE(total > 0 && total < (1ll << 31), "refiner_block_c144: bad tile count");
+    p.total_tiles = (int)total;
+    const int dev = current_device();
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    static bool cfg[64] = {};            // function attributes are per device
+    if (!cfg[dev & 63]) {
+        RB_REQUIRE(cudaFuncSetAttribute(refiner_block_c144_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FS_SMEM) == cudaSuccess, "refiner_block_c144: smem attribute");
+        cfg[dev & 63] = true;
+    }
+    rb::launch_pdl(refiner_block_c144_split_kernel, dim3(p.total_tiles < sms ? p.total_tiles : sms), dim3(FS_THREADS), FS_SMEM, st, map_w[0], map_w[1], map_in, map_out, p);
+    return check_launch("refiner_block_c144_split");
+}
+
 extern "C" int romab200_refiner_block_c144(const rb_refiner_block_c144_args* a, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
     RB_REQUIRE(a->c == FZ_C, "refiner_block_c144: C must be 144 (got %d)", a->c);
-    RB_REQUIRE(a->dtype == RB_F16 || a->dtype == RB_BF16, "refiner_block_c144: 16-bit activations only");
-    RB_REQUIRE(a->ld % 8 == 0 && a->ld >= FZ_C && ((uintptr_t)a->in) % 16 == 0 && ((uintptr_t)a->out) % 16 == 0 && a->in != a->out,
-               "refiner_block_c144: bad activation layout");
+    RB_REQUIRE(a->dtype == RB_F16 || a->dtype == RB_BF16 || a->dtype == RB_F32, "refiner_block_c144: fp16 / bf16 / fp32 activations");
     RB_REQUIRE(a->ld_pw % 8 == 0 && a->ld_pw >= FZ_C && ((uintptr_t)a->pw_weight) % 16 == 0, "refiner_block_c144: bad weight layout");
     static EncodeTiledFnFz enc = nullptr;
     if (!enc) {
@@ -324,6 +630,9 @@ extern "C" int romab200_refiner_block_c144(const rb_refiner_block_c144_args* a, 
                    "refiner_block_c144: cuTensorMapEncodeTiled not available");
         enc = (EncodeTiledFnFz)ptr;
     }
+    if (a->dtype == RB_F32) return refiner_block_c144_split(a, st, enc);
+    RB_REQUIRE(a->ld % 8 == 0 && a->ld >= FZ_C && ((uintptr_t)a->in) % 16 == 0 && ((uintptr_t)a->out) % 16 == 0 && a->in != a->out,
+               "refiner_block_c144: bad activation layout");
     CUtensorMap map;
     cuuint64_t dims[2] = {(cuuint64_t)FZ_C, (cuuint64_t)FZ_C};
     cuuint64_t strides[1] = {(cuuint64_t)a->ld_pw * 2};

@@ -40,6 +40,10 @@ F16S = cabi.RB_F16S
 
 
 class Engine:
+    # parity mode: stride-2 refiner blocks as one fused DW + split-fp16 tcgen05-PW kernel (ROMAB200_FUSED_C144_F32=0: the
+    # un-fused depthwise kernel + split GEMM pair, which computes the same bits)
+    fused_c144_f32 = os.environ.get("ROMAB200_FUSED_C144_F32", "1") != "0"
+
     def __init__(self, matcher_sd, dino_sd, device, precision: str = "fp32"):
         if precision not in PRECISIONS:
             raise ValueError(f"precision must be one of {list(PRECISIONS)}")
@@ -528,6 +532,16 @@ class Engine:
             for blk in R["blocks"]:
                 call("romab200_refiner_block_c144", "rb_refiner_block_c144_args", **{"in": d}, out=t, ld=cp, dw_weight=blk["dw_w"], ldw=cp,
                      dw_bias=blk["dw_b"], pw_weight=blk["pw_w"], ld_pw=cp, pw_bias=blk["pw_b"], batch=D, h=h, w=w, c=c, dtype=self.dt)
+                d, t = t, d
+        elif c == 144 and self.split and self.fused_c144_f32:
+            # parity mode, stride-2 maps: the same fused block on fp32 maps with the split-fp16 pointwise GEMM (bit-identical
+            # to the depthwise kernel + split GEMM pair below, at one read and one write of the map instead of four transfers)
+            if t is None:
+                t = self.buf(f"ref.t.{tag}", (D * h * w, cp), zero=True)
+            for blk in R["blocks"]:
+                call("romab200_refiner_block_c144", "rb_refiner_block_c144_args", **{"in": d}, out=t, ld=cp, dw_weight=blk["dw_w"], ldw=cp,
+                     dw_bias=blk["dw_b"], pw_weight=blk["pw_w"].hi, pw_weight_lo=blk["pw_w"].lo, ld_pw=cp, pw_bias=blk["pw_b"],
+                     batch=D, h=h, w=w, c=c, dtype=cabi.RB_F32)
                 d, t = t, d
         elif self.split:
             # parity mode: fp32 maps; the depthwise kernel writes its result as the RB_F16S A operand of the pointwise GEMM
