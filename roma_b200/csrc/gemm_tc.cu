@@ -105,6 +105,23 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
     for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const float* v) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
+        ::"r"(taddr), "r"(__float_as_uint(v[0])), "r"(__float_as_uint(v[1])), "r"(__float_as_uint(v[2])), "r"(__float_as_uint(v[3])),
+          "r"(__float_as_uint(v[4])), "r"(__float_as_uint(v[5])), "r"(__float_as_uint(v[6])), "r"(__float_as_uint(v[7])),
+          "r"(__float_as_uint(v[8])), "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])),
+          "r"(__float_as_uint(v[12])), "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15])),
+          "r"(__float_as_uint(v[16])), "r"(__float_as_uint(v[17])), "r"(__float_as_uint(v[18])), "r"(__float_as_uint(v[19])),
+          "r"(__float_as_uint(v[20])), "r"(__float_as_uint(v[21])), "r"(__float_as_uint(v[22])), "r"(__float_as_uint(v[23])),
+          "r"(__float_as_uint(v[24])), "r"(__float_as_uint(v[25])), "r"(__float_as_uint(v[26])), "r"(__float_as_uint(v[27])),
+          "r"(__float_as_uint(v[28])), "r"(__float_as_uint(v[29])), "r"(__float_as_uint(v[30])), "r"(__float_as_uint(v[31]))
+        : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
 // 32 consecutive floats of a row vector (bias / LayerScale / residual): 8 x 16-byte loads when possible
 __device__ __forceinline__ void load_row32(const float* __restrict__ p, float* out, bool full, int remaining) {
     if (full && (reinterpret_cast<uintptr_t>(p) & 15) == 0) {
@@ -140,6 +157,7 @@ struct TcParams {
     int tiles_m, tiles_n, total_tiles;
     int64_t sc0, sc1, sr0, sr1, sna0, snb0;
     unsigned long long* clk;      // optional role-time counters (ROMAB200_TC_CLK=1): see tc_clk_dump
+    int band_major;               // tile order: 1 = all N tiles of a row band before the next band, 0 = N-major (see tc_tile_coords)
     int epi_mode;                 // store strategy of the epilogue: 0 = direct row-per-lane stores, 2 = TMA stores from a per-warp staging
                                   // buffer (map_c / map_c_lo), 3 = the same as an fp32 reduce-add (C += tile)
     Epilogue epi;
@@ -152,6 +170,7 @@ __device__ __forceinline__ void clk_add(unsigned long long* clk, int i, long lon
 
 constexpr int TC_BM = 128, TC_BK = 64;
 constexpr int TC_STAGE_WORDS = 512;                // TMA-store staging buffer per epilogue warp: 32 rows x 64 bytes
+constexpr int TC_PARK_WORDS = 1024;                // early-release park buffer per epilogue warp: one 32 x 32 fp32 chunk
 
 template <int BN, bool SPLIT> struct TcCfg {
     // BN = 256: one CTA per SM with 8 epilogue warps; narrower tiles: two CTAs per SM (two MMA-issuing threads keep the
@@ -166,10 +185,12 @@ template <int BN, bool SPLIT> struct TcCfg {
     static constexpr int CTAS_PER_SM = (SPLIT || BN > 128) ? 1 : 2;
     static constexpr int EPI_WARPS = BN > 128 ? 8 : 4;
     static constexpr int THREADS = 64 + 32 * EPI_WARPS;
-    static constexpr int EPI_BYTES = 2 * 256 * 4 + EPI_WARPS * TC_STAGE_WORDS * 4;   // staged bias / column-scale (or norm_b) + per-warp transpose buffers
-    static constexpr int SMEM = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/ + EPI_BYTES;
     static constexpr int ACC_COLS = NOPS * BN;                           // TMEM columns of one accumulator stage
     static constexpr int ACC_STAGES = 2 * ACC_COLS <= 512 ? 2 : 1;       // double-buffered when it fits
+    static constexpr bool EARLY = ACC_STAGES == 1 && BN <= 192;          // epilogue frees the accumulator before its math (tc_epilogue_tile)
+    static constexpr int EPI_BYTES = 2 * 256 * 4 + EPI_WARPS * TC_STAGE_WORDS * 4 +  // staged bias / column-scale (or norm_b) + per-warp transpose buffers
+                                     (EARLY ? EPI_WARPS * TC_PARK_WORDS * 4 : 0);    // + per-warp park buffers
+    static constexpr int SMEM = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/ + EPI_BYTES;
     static constexpr int ACC_TOTAL = ACC_STAGES * ACC_COLS;
     static constexpr int TMEM_COLS = ACC_TOTAL <= 32 ? 32 : (ACC_TOTAL <= 64 ? 64 : (ACC_TOTAL <= 128 ? 128 : (ACC_TOTAL <= 256 ? 256 : 512)));
     static_assert(SMEM <= 232448, "shared memory budget");
@@ -179,10 +200,258 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
+// Tile index -> (m tile, n tile, batch index); the producer and the epilogue of both kernels decode through here.  Consecutive
+// tiles run at about the same time on neighbouring CTAs, so the operand that the order keeps fixed is read from HBM once and shared
+// in L2.  Band-major (the tiles_n tiles of a row band in a row) streams A once and re-reads B per band; N-major streams B once and
+// re-reads A per N tile.  The host picks band-major when A is at least as large as B.
+__device__ __forceinline__ void tc_tile_coords(const TcParams& p, int tile, int& mt, int& nt, int& z) {
+    const int tiles_per_z = p.tiles_m * p.tiles_n;
+    z = tile / tiles_per_z;
+    const int r = tile - z * tiles_per_z;
+    if (p.band_major) { mt = r / p.tiles_n; nt = r - mt * p.tiles_n; }
+    else { nt = r / p.tiles_m; mt = r - nt * p.tiles_m; }
+}
+
+// Math and store of one 32-column chunk of the tile, held in v in the row-per-lane layout of tcgen05.ld (column cb of the tile).
+__device__ __forceinline__ void tc_epilogue_chunk(const TcParams& p, const Epilogue& e, float (&v)[32], int cb, int m0, int n0, int z0, int z1, int q, int lane,
+                                                  int nlim, int m, int64_t orow, bool vec_ok, const float* s_vec0, const float* s_vec1, float* stage,
+                                                  const CUtensorMap* map_c, const CUtensorMap* map_c_lo, bool timing, int& t_math, int& t_store) {
+    const int nb = n0 + cb;
+    const long long tc1 = clock64();
+    // ---- element-wise part in the row-per-lane layout (every branch is warp-uniform) ----
+    if (e.epi == RB_EPI_COSKERNEL) {
+        const float na = m < p.M ? e.norm_a[m] : 1.f;
+        if (e.cos_normalized) {
+            // operands are the L2-normalised rows: c = acc * pn / (pn + eps) = acc * (1 - eps / (pn + eps)).  eps / (pn + eps) is ~1e-9 of
+            // the result, so an approximate reciprocal (2 ulp) leaves the factor correctly rounded in all but exotic cases (pn < 1e-2);
+            // exp(x) = 2^(x log2 e) with x in [-2/T, 0]: the input rounding costs |x log2 e| 2^-24 < 1e-6 relative, an order below the
+            // error of the split contraction itself (8e-6 vs float64).  15 instead of 30 instructions per element: this epilogue, not
+            // the 8-k-block main loop, bounds the launch (ncu: tensor pipe 18 % active).
+            const float k2 = e.inv_t * 1.4426950408889634f;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const float4 b4 = *reinterpret_cast<const float4*>(&s_vec0[cb + 4 * j]);
+                const float bn[4] = {b4.x, b4.y, b4.z, b4.w};
+#pragma unroll
+                for (int t = 0; t < 4; ++t) {
+                    const float pe = fmaf(na, bn[t], e.eps);
+                    float rc;
+                    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc) : "f"(pe));
+                    const float sc = fmaf(-e.eps, rc, 1.0f);
+                    const float x2 = fmaf(v[4 * j + t], sc, -1.0f) * k2;
+                    float r;
+                    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x2));
+                    v[4 * j + t] = r;
+                }
+            }
+            if (e.diag_add != 0.f && m >= nb && m < nb + 32) {     // the diagonal crosses this 32-column chunk in at most one lane per column
+#pragma unroll
+                for (int j = 0; j < 32; ++j) if (m == nb + j) v[j] += e.diag_add;
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+                const int n = nb + j;
+                const float pn = na * s_vec0[cb + j];
+                const float sc = 1.0f / (pn + e.eps);
+                float r = expf((v[j] * sc - 1.0f) * e.inv_t);
+                if (m == n) r += e.diag_add;
+                v[j] = r;
+            }
+        }
+    } else {
+        if (e.alpha != 1.0f) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] *= e.alpha;
+        }
+        if (e.bias) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const float4 b4 = *reinterpret_cast<const float4*>(&s_vec0[cb + 4 * j]);
+                v[4 * j] += b4.x; v[4 * j + 1] += b4.y; v[4 * j + 2] += b4.z; v[4 * j + 3] += b4.w;
+            }
+        }
+        if (e.act == RB_ACT_RELU) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.f);
+        } else if (e.act == RB_ACT_GELU) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = gelu_erf(v[j]);
+        }
+        if (e.col_scale) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const float4 s4 = *reinterpret_cast<const float4*>(&s_vec1[cb + 4 * j]);
+                v[4 * j] *= s4.x; v[4 * j + 1] *= s4.y; v[4 * j + 2] *= s4.z; v[4 * j + 3] *= s4.w;
+            }
+        }
+    }
+    // ---- store ----
+    long long tc2 = clock64();
+    t_math += (int)(tc2 - tc1);
+    if (p.epi_mode >= 2) {
+        // ---- TMA stores: the warp's 32 x 32 chunk goes through its 2 KB staging buffer as [32 rows][64 B] (16-bit output: one
+        // round of 32 columns; fp32 / split pair: two rounds of 16 columns) and leaves with cp.async.bulk.tensor: whole segments,
+        // clipped at the M / N tails by the tensor map, asynchronous to the warp.  Rows that are not stored (the zero border of a
+        // padded map) are written as zeros, which is what they hold already.
+        if (orow < 0) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) v[j] = 0.f;
+        }
+        if (nb + 32 > nlim) {       // the N tail: TMA clips at 16-byte granules, so the pad columns up to the next granule receive zeros
+#pragma unroll
+            for (int j = 0; j < 32; ++j) if (nb + j >= nlim) v[j] = 0.f;
+        }
+        uint8_t* sb = reinterpret_cast<uint8_t*>(stage);
+        const int row0 = m0 + q * 32;
+        if (e.dtype_c == RB_F16 || e.dtype_c == RB_BF16) {
+            if (lane == 0) bulk_wait_read();
+            __syncwarp();
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                uint32_t w[4];
+#pragma unroll
+                for (int t = 0; t < 4; ++t) {
+                    const float lo = v[8 * j + 2 * t], hi = v[8 * j + 2 * t + 1];
+                    if (e.dtype_c == RB_F16) { __half2 hh = __floats2half2_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&hh); }
+                    else { __nv_bfloat162 hh = __floats2bfloat162_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&hh); }
+                }
+                *reinterpret_cast<uint4*>(sb + lane * 64 + 16 * j) = make_uint4(w[0], w[1], w[2], w[3]);
+            }
+            fence_async_smem();
+            __syncwarp();
+            if (lane == 0) { tma_store_4d(map_c, sb, nb, row0, z1, z0); bulk_commit(); }
+        } else {
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                if (nb + 16 * h >= nlim) break;                 // warp-uniform
+                if (lane == 0) bulk_wait_read();
+                __syncwarp();
+                if (e.dtype_c == RB_F32) {
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        *reinterpret_cast<float4*>(sb + lane * 64 + 16 * j) = make_float4(v[16 * h + 4 * j], v[16 * h + 4 * j + 1], v[16 * h + 4 * j + 2], v[16 * h + 4 * j + 3]);
+                } else {                                        // RB_F16S: hi rows at [0, 1 KB), lo rows at [1 KB, 2 KB), 32 B each
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        uint32_t wh[4], wl[4];
+#pragma unroll
+                        for (int t = 0; t < 4; ++t) {
+                            const float x0 = v[16 * h + 8 * j + 2 * t], x1 = v[16 * h + 8 * j + 2 * t + 1];
+                            const __half2 hh = __floats2half2_rn(x0, x1);
+                            const float2 hf = __half22float2(hh);
+                            const __half2 ll = __floats2half2_rn((x0 - hf.x) * 2048.0f, (x1 - hf.y) * 2048.0f);
+                            wh[t] = *reinterpret_cast<const uint32_t*>(&hh); wl[t] = *reinterpret_cast<const uint32_t*>(&ll);
+                        }
+                        *reinterpret_cast<uint4*>(sb + lane * 32 + 16 * j) = make_uint4(wh[0], wh[1], wh[2], wh[3]);
+                        *reinterpret_cast<uint4*>(sb + 1024 + lane * 32 + 16 * j) = make_uint4(wl[0], wl[1], wl[2], wl[3]);
+                    }
+                }
+                fence_async_smem();
+                __syncwarp();
+                if (lane == 0) {
+                    if (e.dtype_c == RB_F32) {
+                        if (p.epi_mode == 3) tma_reduce_add_4d(map_c, sb, nb + 16 * h, row0, z1, z0);
+                        else tma_store_4d(map_c, sb, nb + 16 * h, row0, z1, z0);
+                    } else {
+                        tma_store_4d(map_c, sb, nb + 16 * h, row0, z1, z0);
+                        tma_store_4d(map_c_lo, sb + 1024, nb + 16 * h, row0, z1, z0);
+                    }
+                    bulk_commit();
+                }
+            }
+        }
+    } else if (p.epi_mode == 0) {
+        if (orow >= 0) {
+        const bool full = nb + 32 <= nlim;
+        if (e.epi != RB_EPI_COSKERNEL) {
+        if (e.R) {
+            if (e.dtype_r == RB_F32) {
+                float rv[32];
+                load_row32((const float*)e.R + orow * e.ldr + nb, rv, full, nlim - nb);
+#pragma unroll
+                for (int j = 0; j < 32; ++j) v[j] += rv[j];
+            } else {
+#pragma unroll
+                for (int j = 0; j < 32; ++j)
+                    if (nb + j < nlim) v[j] += load_any(e.R, orow * e.ldr + nb + j, e.dtype_r);
+            }
+        }
+        }
+    if (vec_ok) {
+        if (e.dtype_c == RB_F32) {
+            float* dst = (float*)e.C + orow * e.ldc + nb;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                if (nb + 4 * j + 4 <= nlim) *reinterpret_cast<float4*>(dst + 4 * j) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+                else {
+#pragma unroll
+                    for (int t = 0; t < 4; ++t) if (nb + 4 * j + t < nlim) dst[4 * j + t] = v[4 * j + t];
+                }
+            }
+        } else if (e.dtype_c == RB_F16S) {
+            // split-pair output: hi = fp16(v), lo = fp16((v - hi) * 2^11) into two planes of the same pitch
+            uint16_t* dhi = (uint16_t*)e.C + orow * e.ldc + nb;
+            uint16_t* dlo = (uint16_t*)e.C_lo + orow * e.ldc + nb;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                uint32_t wh[4], wl[4];
+#pragma unroll
+                for (int t = 0; t < 4; ++t) {
+                    const float x0 = v[8 * j + 2 * t], x1 = v[8 * j + 2 * t + 1];
+                    const __half2 h = __floats2half2_rn(x0, x1);
+                    const float2 hf = __half22float2(h);
+                    const __half2 l = __floats2half2_rn((x0 - hf.x) * 2048.0f, (x1 - hf.y) * 2048.0f);
+                    wh[t] = *reinterpret_cast<const uint32_t*>(&h); wl[t] = *reinterpret_cast<const uint32_t*>(&l);
+                }
+                if (nb + 8 * j + 8 <= nlim) {
+                    *reinterpret_cast<uint4*>(dhi + 8 * j) = make_uint4(wh[0], wh[1], wh[2], wh[3]);
+                    *reinterpret_cast<uint4*>(dlo + 8 * j) = make_uint4(wl[0], wl[1], wl[2], wl[3]);
+                } else {
+#pragma unroll
+                    for (int t = 0; t < 8; ++t)
+                        if (nb + 8 * j + t < nlim) {
+                            dhi[8 * j + t] = (uint16_t)(wh[t >> 1] >> (16 * (t & 1)));
+                            dlo[8 * j + t] = (uint16_t)(wl[t >> 1] >> (16 * (t & 1)));
+                        }
+                }
+            }
+        } else {
+            uint16_t* dst = (uint16_t*)e.C + orow * e.ldc + nb;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                uint32_t w[4];
+#pragma unroll
+                for (int t = 0; t < 4; ++t) {
+                    float lo = v[8 * j + 2 * t], hi = v[8 * j + 2 * t + 1];
+                    if (e.dtype_c == RB_F16) { __half2 h = __floats2half2_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&h); }
+                    else { __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&h); }
+                }
+                if (nb + 8 * j + 8 <= nlim) *reinterpret_cast<uint4*>(dst + 8 * j) = make_uint4(w[0], w[1], w[2], w[3]);
+                else {
+#pragma unroll
+                    for (int t = 0; t < 8; ++t)
+                        if (nb + 8 * j + t < nlim) dst[8 * j + t] = (uint16_t)(w[t >> 1] >> (16 * (t & 1)));
+                }
+            }
+        }
+    } else {
+#pragma unroll
+        for (int j = 0; j < 32; ++j)
+            if (nb + j < nlim) store_split_any(e.C, e.C_lo, orow * e.ldc + nb + j, e.dtype_c, v[j]);
+    }
+        }
+    }
+    __syncwarp();
+    if (timing) { t_store += (int)(clock64() - tc2); }
+}
+
 // Epilogue of one 128 x BN accumulator tile by the EPI_WARPS epilogue warps of a CTA (shared by the 1-CTA and the 2-CTA
 // kernels): stage the per-column vectors, wait for the accumulator, tcgen05.ld, fused epilogue, coalesced stores.
 // `tmem_acc` = TMEM address of the tile's main accumulator (lane 0); the cross accumulator of the SPLIT variant sits BN columns
-// further.  (m0, n0) = first row / column of the tile, z0 / z1 = batch indices.
+// further.  (m0, n0) = first row / column of the tile, z0 / z1 = batch indices.  `release()` gives the accumulator back to the MMA
+// thread; EARLY (single-buffered 144 / 192-column split accumulators) calls it as soon as the warp's slice is out of the accumulator,
+// otherwise after the stores.
 //
 // tcgen05.ld hands every lane ONE ROW of the accumulator, so a direct store writes 16-byte pieces of 32 different rows per
 // instruction.  Measured with the role-time counters (ROMAB200_TC_CLK=1, scripts/gemm_clk.py) on the ViT shapes, cycles per
@@ -192,10 +461,10 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 // [32 rows][64 B] and one lane issues cp.async.bulk.tensor stores (UTMASTG; 3.3k / 5.6k cycles, asynchronous to the warp); an
 // in-place fp32 residual (R == C) becomes a TMA reduce-add (UTMAREDG), so the residual stream is never read by the kernel.
 // Row maps other than NONE / PAD_KEEP, mismatched residual operands and unaligned pitches take the direct path.
-template <int BN, bool SPLIT, int EPI_WARPS>
+template <int BN, bool SPLIT, int EPI_WARPS, bool EARLY, class Release>
 __device__ __forceinline__ void tc_epilogue_tile(const TcParams& p, uint32_t tmem_acc, uint64_t* full_bar, uint32_t full_parity, int m0, int n0,
                                                  int z0, int z1, int q, int half, int lane, int et, float* s_vec0, float* s_vec1, float* stage,
-                                                 const CUtensorMap* map_c, const CUtensorMap* map_c_lo) {
+                                                 float* park, const CUtensorMap* map_c, const CUtensorMap* map_c_lo, Release release) {
     const long long t_entry = clock64();
     Epilogue e = p.epi;
     e.C = (char*)e.C + (z0 * p.sc0 + z1 * p.sc1) * dtype_size(e.dtype_c);
@@ -214,8 +483,8 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcParams& p, uint32_t tme
     asm volatile("bar.sync 1, %0;" ::"n"(32 * EPI_WARPS) : "memory");
     const bool timing = p.clk && q == 2 && half == 0 && lane == 0;     // warp 2, lane 0
     const long long tw = clock64();
-    const long long t_pre = tw - t_entry;
-    long long t_ld = 0, t_math = 0, t_store = 0;
+    const int t_pre = (int)(tw - t_entry);
+    int t_ld = 0, t_math = 0, t_store = 0;              // cycles of this tile (warp 2, lane 0): fit 32 bits, spare registers
     mbar_wait(full_bar, full_parity);
     if (timing) clk_add(p.clk, 5, clock64() - tw);
     tc_fence_after();
@@ -225,248 +494,73 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcParams& p, uint32_t tme
     const int es_c = dtype_size(e.dtype_c);
     const bool vec_ok = (e.ldc * es_c) % 16 == 0 && (reinterpret_cast<uintptr_t>(e.C) % 16 == 0) &&
                         (e.dtype_c != RB_F16S || reinterpret_cast<uintptr_t>(e.C_lo) % 16 == 0);
-#pragma unroll 1
-    for (int cb = half * 32; cb < BN; cb += 8 * EPI_WARPS) {
-        if (n0 + cb >= nlim) break;                     // warp-uniform
-        float v[32];
-        const long long tc0 = clock64();
-        // all 32 lanes take part in the TMEM loads (.sync.aligned); rows that are not stored are masked in the store phase
+    // one 32-column chunk of the accumulator (both accumulators of the SPLIT variant, combined); all 32 lanes take part in the TMEM
+    // loads (.sync.aligned); rows that are not stored are masked in the store phase
+    auto load_chunk = [&](int cb, float (&v)[32]) {
         tmem_ld32(tmem_acc + ((uint32_t)(q * 32) << 16) + cb, v);
         if constexpr (SPLIT) {
             float w[32];
             tmem_ld32(tmem_acc + ((uint32_t)(q * 32) << 16) + BN + cb, w);
-    #pragma unroll
+#pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = fmaf(w[j], 1.0f / 2048.0f, v[j]);
         }
-        const int nb = n0 + cb;
-        const long long tc1 = clock64();
-        t_ld += tc1 - tc0;
-        // ---- element-wise part in the row-per-lane layout (every branch is warp-uniform) ----
-        if (e.epi == RB_EPI_COSKERNEL) {
-            const float na = m < p.M ? e.norm_a[m] : 1.f;
-            if (e.cos_normalized) {
-                // operands are the L2-normalised rows: c = acc * pn / (pn + eps) = acc * (1 - eps / (pn + eps)).  eps / (pn + eps) is ~1e-9 of
-                // the result, so an approximate reciprocal (2 ulp) leaves the factor correctly rounded in all but exotic cases (pn < 1e-2);
-                // exp(x) = 2^(x log2 e) with x in [-2/T, 0]: the input rounding costs |x log2 e| 2^-24 < 1e-6 relative, an order below the
-                // error of the split contraction itself (8e-6 vs float64).  15 instead of 30 instructions per element: this epilogue, not
-                // the 8-k-block main loop, bounds the launch (ncu: tensor pipe 18 % active).
-                const float k2 = e.inv_t * 1.4426950408889634f;
-    #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float4 b4 = *reinterpret_cast<const float4*>(&s_vec0[cb + 4 * j]);
-                    const float bn[4] = {b4.x, b4.y, b4.z, b4.w};
-    #pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        const float pe = fmaf(na, bn[t], e.eps);
-                        float rc;
-                        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc) : "f"(pe));
-                        const float sc = fmaf(-e.eps, rc, 1.0f);
-                        const float x2 = fmaf(v[4 * j + t], sc, -1.0f) * k2;
-                        float r;
-                        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x2));
-                        v[4 * j + t] = r;
-                    }
-                }
-                if (e.diag_add != 0.f && m >= nb && m < nb + 32) {     // the diagonal crosses this 32-column chunk in at most one lane per column
-    #pragma unroll
-                    for (int j = 0; j < 32; ++j) if (m == nb + j) v[j] += e.diag_add;
-                }
-            } else {
-    #pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const int n = nb + j;
-                    const float pn = na * s_vec0[cb + j];
-                    const float sc = 1.0f / (pn + e.eps);
-                    float r = expf((v[j] * sc - 1.0f) * e.inv_t);
-                    if (m == n) r += e.diag_add;
-                    v[j] = r;
-                }
-            }
-        } else {
-            if (e.alpha != 1.0f) {
-    #pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] *= e.alpha;
-            }
-            if (e.bias) {
-    #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float4 b4 = *reinterpret_cast<const float4*>(&s_vec0[cb + 4 * j]);
-                    v[4 * j] += b4.x; v[4 * j + 1] += b4.y; v[4 * j + 2] += b4.z; v[4 * j + 3] += b4.w;
-                }
-            }
-            if (e.act == RB_ACT_RELU) {
-    #pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.f);
-            } else if (e.act == RB_ACT_GELU) {
-    #pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = gelu_erf(v[j]);
-            }
-            if (e.col_scale) {
-    #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const float4 s4 = *reinterpret_cast<const float4*>(&s_vec1[cb + 4 * j]);
-                    v[4 * j] *= s4.x; v[4 * j + 1] *= s4.y; v[4 * j + 2] *= s4.z; v[4 * j + 3] *= s4.w;
-                }
-            }
-        }
-        // ---- store ----
-        long long tc2 = clock64();
-        t_math += tc2 - tc1;
-        if (p.epi_mode >= 2) {
-            // ---- TMA stores: the warp's 32 x 32 chunk goes through its 2 KB staging buffer as [32 rows][64 B] (16-bit output: one
-            // round of 32 columns; fp32 / split pair: two rounds of 16 columns) and leaves with cp.async.bulk.tensor: whole segments,
-            // clipped at the M / N tails by the tensor map, asynchronous to the warp.  Rows that are not stored (the zero border of a
-            // padded map) are written as zeros, which is what they hold already.
-            if (orow < 0) {
-    #pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = 0.f;
-            }
-            if (nb + 32 > nlim) {       // the N tail: TMA clips at 16-byte granules, so the pad columns up to the next granule receive zeros
-    #pragma unroll
-                for (int j = 0; j < 32; ++j) if (nb + j >= nlim) v[j] = 0.f;
-            }
-            uint8_t* sb = reinterpret_cast<uint8_t*>(stage);
-            const int row0 = m0 + q * 32;
-            if (e.dtype_c == RB_F16 || e.dtype_c == RB_BF16) {
-                if (lane == 0) bulk_wait_read();
-                __syncwarp();
-    #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    uint32_t w[4];
-    #pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        const float lo = v[8 * j + 2 * t], hi = v[8 * j + 2 * t + 1];
-                        if (e.dtype_c == RB_F16) { __half2 hh = __floats2half2_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&hh); }
-                        else { __nv_bfloat162 hh = __floats2bfloat162_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&hh); }
-                    }
-                    *reinterpret_cast<uint4*>(sb + lane * 64 + 16 * j) = make_uint4(w[0], w[1], w[2], w[3]);
-                }
-                fence_async_smem();
-                __syncwarp();
-                if (lane == 0) { tma_store_4d(map_c, sb, nb, row0, z1, z0); bulk_commit(); }
-            } else {
-    #pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    if (nb + 16 * h >= nlim) break;                 // warp-uniform
-                    if (lane == 0) bulk_wait_read();
-                    __syncwarp();
-                    if (e.dtype_c == RB_F32) {
-    #pragma unroll
-                        for (int j = 0; j < 4; ++j)
-                            *reinterpret_cast<float4*>(sb + lane * 64 + 16 * j) = make_float4(v[16 * h + 4 * j], v[16 * h + 4 * j + 1], v[16 * h + 4 * j + 2], v[16 * h + 4 * j + 3]);
-                    } else {                                        // RB_F16S: hi rows at [0, 1 KB), lo rows at [1 KB, 2 KB), 32 B each
-    #pragma unroll
-                        for (int j = 0; j < 2; ++j) {
-                            uint32_t wh[4], wl[4];
-    #pragma unroll
-                            for (int t = 0; t < 4; ++t) {
-                                const float x0 = v[16 * h + 8 * j + 2 * t], x1 = v[16 * h + 8 * j + 2 * t + 1];
-                                const __half2 hh = __floats2half2_rn(x0, x1);
-                                const float2 hf = __half22float2(hh);
-                                const __half2 ll = __floats2half2_rn((x0 - hf.x) * 2048.0f, (x1 - hf.y) * 2048.0f);
-                                wh[t] = *reinterpret_cast<const uint32_t*>(&hh); wl[t] = *reinterpret_cast<const uint32_t*>(&ll);
-                            }
-                            *reinterpret_cast<uint4*>(sb + lane * 32 + 16 * j) = make_uint4(wh[0], wh[1], wh[2], wh[3]);
-                            *reinterpret_cast<uint4*>(sb + 1024 + lane * 32 + 16 * j) = make_uint4(wl[0], wl[1], wl[2], wl[3]);
-                        }
-                    }
-                    fence_async_smem();
-                    __syncwarp();
-                    if (lane == 0) {
-                        if (e.dtype_c == RB_F32) {
-                            if (p.epi_mode == 3) tma_reduce_add_4d(map_c, sb, nb + 16 * h, row0, z1, z0);
-                            else tma_store_4d(map_c, sb, nb + 16 * h, row0, z1, z0);
-                        } else {
-                            tma_store_4d(map_c, sb, nb + 16 * h, row0, z1, z0);
-                            tma_store_4d(map_c_lo, sb + 1024, nb + 16 * h, row0, z1, z0);
-                        }
-                        bulk_commit();
-                    }
-                }
-            }
-        } else if (p.epi_mode == 0) {
-            if (orow >= 0) {
-            const bool full = nb + 32 <= nlim;
-            if (e.epi != RB_EPI_COSKERNEL) {
-            if (e.R) {
-                if (e.dtype_r == RB_F32) {
-                    float rv[32];
-                    load_row32((const float*)e.R + orow * e.ldr + nb, rv, full, nlim - nb);
-    #pragma unroll
-                    for (int j = 0; j < 32; ++j) v[j] += rv[j];
+    };
+    if constexpr (EARLY) {
+        // single-buffered accumulator (split tiles of 144 / 192 columns): the warp first takes its whole row slice (at most 3 chunks of
+        // 32 columns) out of the accumulator and gives it back, so that the math and the stores overlap the MMAs of the next tile.  The
+        // combined chunks wait in TMEM columns the accumulator does not use (2 * BN .. 511: 64 per warp) and, the third one, in the
+        // warp's 4 KB park buffer in shared memory.  (Holding them in registers spills: 10 warps leave 168 per thread.)  Park layout:
+        // lane = row, its eight 16-byte granules XOR-swizzled by lane & 7, which keeps the accesses free of bank conflicts.
+        constexpr int NCH = (BN + 8 * EPI_WARPS - 1) / (8 * EPI_WARPS);
+        static_assert(NCH <= 3 && 2 * BN + 2 * 64 <= 512, "early release: two chunks per warp in spare TMEM columns, one in shared memory");
+        const uint32_t spare = tmem_acc + ((uint32_t)(q * 32) << 16) + 2 * BN + half * 64;
+        float4* prow = reinterpret_cast<float4*>(park) + lane * 8;
+        const long long tc0 = clock64();
+#pragma unroll
+        for (int c = 0; c < NCH; ++c) {
+            const int cb = half * 32 + c * 8 * EPI_WARPS;
+            if (cb < BN && n0 + cb < nlim) {                   // warp-uniform
+                float v[32];
+                load_chunk(cb, v);
+                if (c < 2) {
+                    tmem_st32(spare + 32 * c, v);
                 } else {
-    #pragma unroll
-                    for (int j = 0; j < 32; ++j)
-                        if (nb + j < nlim) v[j] += load_any(e.R, orow * e.ldr + nb + j, e.dtype_r);
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) prow[j ^ (lane & 7)] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
                 }
-            }
-            }
-        if (vec_ok) {
-            if (e.dtype_c == RB_F32) {
-                float* dst = (float*)e.C + orow * e.ldc + nb;
-    #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    if (nb + 4 * j + 4 <= nlim) *reinterpret_cast<float4*>(dst + 4 * j) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-                    else {
-    #pragma unroll
-                        for (int t = 0; t < 4; ++t) if (nb + 4 * j + t < nlim) dst[4 * j + t] = v[4 * j + t];
-                    }
-                }
-            } else if (e.dtype_c == RB_F16S) {
-                // split-pair output: hi = fp16(v), lo = fp16((v - hi) * 2^11) into two planes of the same pitch
-                uint16_t* dhi = (uint16_t*)e.C + orow * e.ldc + nb;
-                uint16_t* dlo = (uint16_t*)e.C_lo + orow * e.ldc + nb;
-    #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    uint32_t wh[4], wl[4];
-    #pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        const float x0 = v[8 * j + 2 * t], x1 = v[8 * j + 2 * t + 1];
-                        const __half2 h = __floats2half2_rn(x0, x1);
-                        const float2 hf = __half22float2(h);
-                        const __half2 l = __floats2half2_rn((x0 - hf.x) * 2048.0f, (x1 - hf.y) * 2048.0f);
-                        wh[t] = *reinterpret_cast<const uint32_t*>(&h); wl[t] = *reinterpret_cast<const uint32_t*>(&l);
-                    }
-                    if (nb + 8 * j + 8 <= nlim) {
-                        *reinterpret_cast<uint4*>(dhi + 8 * j) = make_uint4(wh[0], wh[1], wh[2], wh[3]);
-                        *reinterpret_cast<uint4*>(dlo + 8 * j) = make_uint4(wl[0], wl[1], wl[2], wl[3]);
-                    } else {
-    #pragma unroll
-                        for (int t = 0; t < 8; ++t)
-                            if (nb + 8 * j + t < nlim) {
-                                dhi[8 * j + t] = (uint16_t)(wh[t >> 1] >> (16 * (t & 1)));
-                                dlo[8 * j + t] = (uint16_t)(wl[t >> 1] >> (16 * (t & 1)));
-                            }
-                    }
-                }
-            } else {
-                uint16_t* dst = (uint16_t*)e.C + orow * e.ldc + nb;
-    #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    uint32_t w[4];
-    #pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        float lo = v[8 * j + 2 * t], hi = v[8 * j + 2 * t + 1];
-                        if (e.dtype_c == RB_F16) { __half2 h = __floats2half2_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&h); }
-                        else { __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi); w[t] = *reinterpret_cast<uint32_t*>(&h); }
-                    }
-                    if (nb + 8 * j + 8 <= nlim) *reinterpret_cast<uint4*>(dst + 8 * j) = make_uint4(w[0], w[1], w[2], w[3]);
-                    else {
-    #pragma unroll
-                        for (int t = 0; t < 8; ++t)
-                            if (nb + 8 * j + t < nlim) dst[8 * j + t] = (uint16_t)(w[t >> 1] >> (16 * (t & 1)));
-                    }
-                }
-            }
-        } else {
-    #pragma unroll
-            for (int j = 0; j < 32; ++j)
-                if (nb + j < nlim) store_split_any(e.C, e.C_lo, orow * e.ldc + nb + j, e.dtype_c, v[j]);
-        }
             }
         }
-        __syncwarp();
-        if (timing) { t_store += clock64() - tc2; }
+        tmem_st_wait();
+        release();
+        t_ld = (int)(clock64() - tc0);
+#pragma unroll
+        for (int c = 0; c < NCH; ++c) {
+            const int cb = half * 32 + c * 8 * EPI_WARPS;
+            if (cb < BN && n0 + cb < nlim) {
+                float v[32];
+                if (c < 2) {
+                    tmem_ld32(spare + 32 * c, v);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const float4 t = prow[j ^ (lane & 7)];
+                        v[4 * j] = t.x; v[4 * j + 1] = t.y; v[4 * j + 2] = t.z; v[4 * j + 3] = t.w;
+                    }
+                }
+                tc_epilogue_chunk(p, e, v, cb, m0, n0, z0, z1, q, lane, nlim, m, orow, vec_ok, s_vec0, s_vec1, stage, map_c, map_c_lo, timing, t_math, t_store);
+            }
+        }
+    } else {
+#pragma unroll 1
+        for (int cb = half * 32; cb < BN; cb += 8 * EPI_WARPS) {
+            if (n0 + cb >= nlim) break;                     // warp-uniform
+            float v[32];
+            const long long tc0 = clock64();
+            load_chunk(cb, v);
+            t_ld += (int)(clock64() - tc0);
+            tc_epilogue_chunk(p, e, v, cb, m0, n0, z0, z1, q, lane, nlim, m, orow, vec_ok, s_vec0, s_vec1, stage, map_c, map_c_lo, timing, t_math, t_store);
+        }
+        release();
     }
     if (timing) { clk_add(p.clk, 11, t_pre); clk_add(p.clk, 12, t_ld); clk_add(p.clk, 13, t_math); clk_add(p.clk, 14, t_store); }
     __syncwarp();
@@ -478,8 +572,8 @@ __device__ __forceinline__ void tc_epilogue_drain(const TcParams& p, int lane) {
     __syncwarp();
 }
 
-// Persistent kernel: every CTA walks tiles t = blockIdx.x, blockIdx.x + gridDim.x, ... (m fastest, so CTAs that run
-// together share the same weight tile in L2).  The accumulator is double-buffered in TMEM when it fits: the MMA warp
+// Persistent kernel: every CTA walks tiles t = blockIdx.x, blockIdx.x + gridDim.x, ... in the order of tc_tile_coords (CTAs that
+// run together share the larger operand's tiles in L2).  The accumulator is double-buffered in TMEM when it fits: the MMA warp
 // starts the next tile while the epilogue warps drain the previous one.
 template <int BN, bool SPLIT>
 __global__ void __launch_bounds__(TcCfg<BN, SPLIT>::THREADS, 1)
@@ -499,10 +593,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty_bar + 2);
     float* s_vec0 = reinterpret_cast<float*>(smem + STAGES * Cfg::STAGE_BYTES + 256);   // bias      | norm_b
     float* s_vec1 = s_vec0 + 256;                                                        // col_scale
+    float* park = s_vec1 + 256 + Cfg::EPI_WARPS * TC_STAGE_WORDS + (threadIdx.x / 32 - 2) * TC_PARK_WORDS;   // this epilogue warp's (Cfg::EARLY)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int kblocks = (p.K + TC_BK - 1) / TC_BK;
-    const int tiles_per_z = p.tiles_m * p.tiles_n;
 
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
@@ -525,8 +619,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             uint32_t it = 0;
             long long w_empty = 0; const long long t_begin = clock64();
             for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
-                const int z = tile / tiles_per_z, r = tile - z * tiles_per_z;
-                const int nt = r / p.tiles_m, mt = r - nt * p.tiles_m;
+                int mt, nt, z;
+                tc_tile_coords(p, tile, mt, nt, z);
                 const int m0 = mt * TC_BM, n0 = nt * BN, z0 = z / p.batch1, z1 = z - z0 * p.batch1;
                 for (int kb = 0; kb < kblocks; ++kb, ++it) {
                     const int s = it % STAGES;
@@ -618,15 +712,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         const int et = threadIdx.x - 64;                      // 0..255 among the epilogue threads
         uint32_t tcount = 0;
         for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++tcount) {
-            const int z = tile / tiles_per_z, r = tile - z * tiles_per_z;
-            const int nt = r / p.tiles_m, mt = r - nt * p.tiles_m;
+            int mt, nt, z;
+            tc_tile_coords(p, tile, mt, nt, z);
             const int m0 = mt * TC_BM, n0 = nt * BN, z0 = z / p.batch1, z1 = z - z0 * p.batch1;
             const uint32_t acc = tcount % Cfg::ACC_STAGES, acc_ph = (tcount / Cfg::ACC_STAGES) & 1;
             const long long te = clock64();
-            tc_epilogue_tile<BN, SPLIT, Cfg::EPI_WARPS>(p, tmem_base + acc * Cfg::ACC_COLS, &tmem_full_bar[acc], acc_ph, m0, n0, z0, z1, q, half, lane, et, s_vec0, s_vec1, s_vec1 + 256 + (warp - 2) * TC_STAGE_WORDS, &map_c, &map_c_lo);
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tmem_empty_bar[acc]);
+            auto release = [&] { tc_fence_before(); __syncwarp(); if (lane == 0) mbar_arrive(&tmem_empty_bar[acc]); };
+            tc_epilogue_tile<BN, SPLIT, Cfg::EPI_WARPS, Cfg::EARLY>(p, tmem_base + acc * Cfg::ACC_COLS, &tmem_full_bar[acc], acc_ph, m0, n0, z0, z1, q, half, lane, et,
+                                                                  s_vec0, s_vec1, s_vec1 + 256 + (warp - 2) * TC_STAGE_WORDS, park, &map_c, &map_c_lo, release);
             if (warp == 2 && lane == 0) clk_add(p.clk, 6, clock64() - te);
         }
         tc_epilogue_drain(p, lane);
@@ -689,15 +782,19 @@ template <int BN, bool SPLIT> struct TcPairCfg {
     static constexpr int B_BYTES = (BN / 2) * TC_BK * 2;                 // this CTA's half of the B tile
     static constexpr int STAGE_BYTES = NOPS * (A_BYTES + B_BYTES);
     static constexpr int EPI_WARPS = 8;
-    static constexpr int EPI_BYTES = 2 * 256 * 4 + EPI_WARPS * TC_STAGE_WORDS * 4;
-    static constexpr int STAGES = (232448 - 1024 - 256 - EPI_BYTES) / STAGE_BYTES > 6 ? 6 : (232448 - 1024 - 256 - EPI_BYTES) / STAGE_BYTES;
+    static constexpr int VEC_BYTES = 2 * 256 * 4 + EPI_WARPS * TC_STAGE_WORDS * 4;
+    static constexpr int STAGES = (232448 - 1024 - 256 - VEC_BYTES) / STAGE_BYTES > 6 ? 6 : (232448 - 1024 - 256 - VEC_BYTES) / STAGE_BYTES;
     static constexpr int THREADS = 64 + 32 * EPI_WARPS;
-    static constexpr int SMEM = STAGES * STAGE_BYTES + 1024 + 256 + EPI_BYTES;
     static constexpr int ACC_COLS = NOPS * BN;
     static constexpr int ACC_STAGES = 2 * ACC_COLS <= 512 ? 2 : 1;
     static constexpr int ACC_TOTAL = ACC_STAGES * ACC_COLS;
     static constexpr int TMEM_COLS = ACC_TOTAL <= 256 ? 256 : 512;
+    // early release (tc_epilogue_tile) needs spare TMEM columns and a 4 KB park buffer per epilogue warp: 192 has both, 256 neither
+    static constexpr bool EARLY = ACC_STAGES == 1 && BN <= 192;
+    static constexpr int EPI_BYTES = VEC_BYTES + (EARLY ? EPI_WARPS * TC_PARK_WORDS * 4 : 0);
+    static constexpr int SMEM = STAGES * STAGE_BYTES + 1024 + 256 + EPI_BYTES;
     static_assert(BN % 32 == 0 && BN <= 256 && STAGES >= 2, "pair tile");
+    static_assert(SMEM <= 232448, "shared memory budget");
 };
 
 // Persistent CTA-pair kernel: cluster c walks pair tiles t = c, c + #clusters, ...  Rank 0 (the leader) issues every MMA
@@ -722,12 +819,12 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty_bar + 2);
     float* s_vec0 = reinterpret_cast<float*>(smem + STAGES * Cfg::STAGE_BYTES + 256);
     float* s_vec1 = s_vec0 + 256;
+    float* park = s_vec1 + 256 + Cfg::EPI_WARPS * TC_STAGE_WORDS + (threadIdx.x / 32 - 2) * TC_PARK_WORDS;   // this epilogue warp's (Cfg::EARLY)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
     const int cid = blockIdx.x >> 1, nclusters = gridDim.x >> 1;
     const int kblocks = (p.K + TC_BK - 1) / TC_BK;
-    const int tiles_per_z = p.tiles_m * p.tiles_n;
 
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
@@ -748,8 +845,8 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
             uint32_t it = 0;
             long long w_empty = 0; const long long t_begin = clock64();
             for (int tile = cid; tile < p.total_tiles; tile += nclusters) {
-                const int z = tile / tiles_per_z, r = tile - z * tiles_per_z;
-                const int nt = r / p.tiles_m, mt = r - nt * p.tiles_m;
+                int mt, nt, z;
+                tc_tile_coords(p, tile, mt, nt, z);
                 const int m0 = mt * (2 * TC_BM) + (int)rank * TC_BM, n0 = nt * BN + (int)rank * (BN / 2);
                 const int z0 = z / p.batch1, z1 = z - z0 * p.batch1;
                 for (int kb = 0; kb < kblocks; ++kb, ++it) {
@@ -828,15 +925,14 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         const int et = threadIdx.x - 64;
         uint32_t tcount = 0;
         for (int tile = cid; tile < p.total_tiles; tile += nclusters, ++tcount) {
-            const int z = tile / tiles_per_z, r = tile - z * tiles_per_z;
-            const int nt = r / p.tiles_m, mt = r - nt * p.tiles_m;
+            int mt, nt, z;
+            tc_tile_coords(p, tile, mt, nt, z);
             const int m0 = mt * (2 * TC_BM) + (int)rank * TC_BM, n0 = nt * BN, z0 = z / p.batch1, z1 = z - z0 * p.batch1;
             const uint32_t acc = tcount % Cfg::ACC_STAGES, acc_ph = (tcount / Cfg::ACC_STAGES) & 1;
             const long long te = clock64();
-            tc_epilogue_tile<BN, SPLIT, Cfg::EPI_WARPS>(p, tmem_base + acc * Cfg::ACC_COLS, &tmem_full_bar[acc], acc_ph, m0, n0, z0, z1, q, half, lane, et, s_vec0, s_vec1, s_vec1 + 256 + (warp - 2) * TC_STAGE_WORDS, &map_c, &map_c_lo);
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cta(&tmem_empty_bar[acc], 0);
+            auto release = [&] { tc_fence_before(); __syncwarp(); if (lane == 0) mbar_arrive_cta(&tmem_empty_bar[acc], 0); };
+            tc_epilogue_tile<BN, SPLIT, Cfg::EPI_WARPS, Cfg::EARLY>(p, tmem_base + acc * Cfg::ACC_COLS, &tmem_full_bar[acc], acc_ph, m0, n0, z0, z1, q, half, lane, et,
+                                                                  s_vec0, s_vec1, s_vec1 + 256 + (warp - 2) * TC_STAGE_WORDS, park, &map_c, &map_c_lo, release);
             if (warp == 2 && lane == 0 && rank == 0) clk_add(p.clk, 6, clock64() - te);
         }
         tc_epilogue_drain(p, lane);
@@ -1021,6 +1117,9 @@ int gemm_tc(const rb_gemm_args* a, cudaStream_t stream) {
     p.trans_b = a->trans_b; p.is_bf16 = a->dtype_ab == RB_BF16;
     p.sc0 = a->sc0; p.sc1 = a->sc1; p.sr0 = a->sr0; p.sr1 = a->sr1; p.sna0 = a->sna0; p.snb0 = a->snb0;
     p.epi = make_epilogue(a);
+    // A (M x K) at least as large as B (N x K): walk row bands, so that A streams from HBM once (refiner pointwise convolutions: up to
+    // 93312 x 569 against 569 x 569); otherwise N-major, which re-reads the smaller A
+    p.band_major = a->M >= a->N;
     p.clk = tc_clk_buffer();
     { static const int em = [] { const char* e = getenv("ROMAB200_GEMM_EPI"); return e && atoi(e) == 0 ? 0 : 2; }(); p.epi_mode = em; }
     if (p.ntaps > 1) {
@@ -1046,7 +1145,9 @@ int gemm_tc(const rb_gemm_args* a, cudaStream_t stream) {
     if (BN > 128 && ((int64_t)((a->M + 127) / 128) * ((a->N + BN - 1) / BN) * zdim) < 100) BN = 128;
     // CTA-pair candidates: all tiles of a launch take the same time, so the launch costs ceil(tiles / SM pairs) waves of a tile whose time
     // grows with BN.  When the 256-wide choice ends in a mostly empty last wave, 192-wide tiles finish earlier (ViT qkv, 3202 x 3072:
-    // 156 tiles = 3 waves of 256 columns against 208 tiles = 3 waves of 192); a 5 % handicap keeps the wider tile on ties.
+    // 156 tiles = 3 waves of 256 columns against 208 tiles = 3 waves of 192); a 5 % handicap keeps the wider tile on ties.  (Split ViT
+    // fc1, 3202 x 4096, ties at 4 waves of 192 against 3 of 256: 192 with early release is faster alone, 86 against 93 us, but slower
+    // inside the step, 2.29 against 2.13 ms, where it shares the GPU with the CNN branch; so the tie stays with 256.)
     if (!a->trans_b && BN == 256 && pair_mode() && wave_rule()) {
         const long long mt = (long long)((a->M + 255) / 256) * zdim, units = sm_count() / 2 > 0 ? sm_count() / 2 : 1;
         auto cost = [&](int bn) { const long long t = mt * ((a->N + bn - 1) / bn); return (t + units - 1) / units * bn; };
